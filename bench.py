@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...     # the reference algorithm (oracle port) on the host cores
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR     # + what the last timed step computed, as DIR/*.npy
 
 Workload (BASELINE.json config 3, "C3"): CelebA-128 deblurring, Unet(dim 64, mults (1,2,4,8), 3 channels),
 T=200, Exponential_reflect k=15 std=0.01, x0_step_down; synthetic U(-1,1) images, random-init weights.
@@ -170,6 +171,23 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_SAMPLE = 1 << 21      # weights drawn per network by --dump-outputs: <= 8 MB of float32 out of the 226 MB of config 3
+
+
+def dump_outputs(out_dir, loss, nets):
+    """writes the loss of the last timed step and, for every net, a fixed seeded sample of its weights after that step (all
+    tensors of state_dict() flattened in key order: the reference layout, whatever layout the engine keeps internally)"""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'loss.npy'), np.asarray([loss.item()], dtype=np.float32))
+    for name, net in nets.items():
+        with torch.no_grad():
+            flat = torch.cat([v.reshape(-1).float() for v in net.state_dict().values()])
+            idx = np.unique(np.random.RandomState(0).randint(0, flat.numel(), DUMP_SAMPLE))
+            np.save(os.path.join(out_dir, name + '.npy'), flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy())
+
+
 def _timed_loop(fn, n, sync):
     import torch
     sync()
@@ -195,7 +213,12 @@ def main():
     ap.add_argument('--no-autotune', action='store_true', help='accepted for compatibility; there is no start-up tuning any more')
     ap.add_argument('--reference-device', default='cpu', choices=['cpu', 'cuda'],
                     help="--impl reference only: 'cpu' (the contract) or 'cuda' = the same eager-PyTorch restatement on the GPU (informational)")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed training step computed (its loss, seeded samples of the weights and EMA weights '
+                         'after it) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -249,8 +272,10 @@ def main():
             ms = tt.item()
         return ms
 
+    last_loss = [None]
+
     def step_resident(s):
-        trainer.train_step(batches=[resident[(s * A + i) % (nb * A)] for i in range(A)])
+        last_loss[0] = trainer.train_step(batches=[resident[(s * A + i) % (nb * A)] for i in range(A)])
         trainer.step += 1
 
     losses = []
@@ -280,6 +305,8 @@ def main():
     _lib.reset_launch_count()
     ms = timed(step_resident, K)
     launches = _lib.launch_count()
+    if args.dump_outputs and rank == 0:     # before any later step moves the weights on
+        dump_outputs(args.dump_outputs, last_loss[0], {'weights': unet, 'ema_weights': trainer.ema_model.denoise_fn})
     for s in range(2):                      # untimed: first use of the pinned batches / loss buffers / events of the end-to-end path
         wl = trainer.train_step(batches=[host[(s * A + i) % (nb * A)] for i in range(A)])
         trainer.step += 1

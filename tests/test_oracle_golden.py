@@ -3,7 +3,6 @@
 import os
 import numpy as np
 import torch
-import pytest
 
 import unet_oracle as UO
 import deblur_oracle as DO
@@ -200,27 +199,19 @@ def test_model2_oracle_matches_reference():
     assert rel(xt, g['s_xt']) < 1e-5 and rel(dr, g['s_dr']) < 1e-5 and rel(img, g['s_img']) < 1e-4
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference'), reason='reference only in build container')
-def test_oracle_matches_live_reference_config1_mnist():
-    """BASELINE config 1: MNIST-shaped 1x32x32, T=20, k=11, sigma=7, Constant, B=4, full-size Unet."""
-    import ref_shim, io, contextlib
-    m = ref_shim.import_reference('deblurring-diffusion-pytorch', 'deblurring_diffusion_pytorch')
-    torch.manual_seed(0)
-    with contextlib.redirect_stdout(io.StringIO()):
-        unet = m.Unet(dim=64, dim_mults=(1, 2, 4, 8), channels=1)
-    gd = m.GaussianDiffusion(unet, image_size=32, device_of_kernel='cpu', channels=1, timesteps=20,
-                             kernel_std=7.0, kernel_size=11, blur_routine='Constant', loss_type='l1')
-    torch.manual_seed(1234)
-    x = torch.rand(4, 1, 32, 32) * 2 - 1
-    t = torch.randint(0, 20, (4,))
-    with torch.no_grad():
-        ref_loss = gd.p_losses(x, t)
-    sd = unet.state_dict()
+def test_oracle_matches_reference_config1_mnist():
+    """BASELINE config 1: MNIST-shaped 1x32x32, T=20, k=11, sigma=7, Constant, B=4, full-size Unet, against the reference's
+    loss and network output (tests/golden/gen_golden_config1.py; the weights are rebuilt from their seed)."""
+    g = load('config1_mnist')
+    sd = UO.make_unet_state_dict(64, (1, 2, 4, 8), 1, seed=0)
     o = DO.DeblurOracle(lambda a, b: UO.unet_forward(sd, a, b), image_size=32, channels=1, timesteps=20,
                         kernel_std=7.0, kernel_size=11, blur_routine='Constant')
+    x, t = g['x'], g['t']
     with torch.no_grad():
         loss = o.p_losses(x, t)
-    assert abs(loss.item() - ref_loss.item()) < 1e-5
+        y = UO.unet_forward(sd, o.q_sample(x, t), t)
+    assert abs(loss.item() - g['loss'].item()) < 1e-5
+    assert rel(y, g['y']) < 1e-5
 
 
 def _small_fn():
@@ -300,7 +291,13 @@ def test_model2_oracle_gradients_match_reference():
     n = 0
     for k, v in gg.items():
         if k.startswith('grad:'):
-            assert rel(sd[k[5:]].grad, v) < 3e-5, k
+            if v.abs().max() < 1e-7:
+                # zero in exact arithmetic (a per-channel shift in front of a one-channel GroupNorm group: conv1.bias / temb_proj
+                # at ch = 32; the key bias in front of a row softmax): round-off on both sides, whose pattern changes with the
+                # number of CPU threads, so the check is absolute, as in tests/test_model2_host_logic.py
+                assert sd[k[5:]].grad.abs().max() < 1e-7, k
+            else:
+                assert rel(sd[k[5:]].grad, v) < 3e-5, k
             n += 1
         elif k.startswith('gsub:'):
             gr = sd[k[5:]].grad.reshape(-1)
